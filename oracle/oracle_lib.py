@@ -28,8 +28,9 @@ _i32p = C.POINTER(C.c_int32)
 
 
 def build(force: bool = False) -> None:
-    """Compile the oracle (port always; _ref only where /root/reference exists)."""
-    targets = ["port"]
+    """Compile the oracle: the restatement and the product's adapter libraries always, the verbatim reference build (_ref)
+    only where the reference tree exists."""
+    targets = ["port", "adapt"]
     if os.path.exists(os.path.join(REFERENCE_ROOT, "src", "ORBextractor.cc")):
         targets.append("ref")
     if force:

@@ -45,15 +45,12 @@ def test_adapters_compile_and_link(tmp_path):
 
 def test_matcher_adapter_library_builds_and_exports_the_reference_entry_points():
     """integration/ORBmatcher_borb.cc (every ORBmatcher method through include/borb_matcher_adapters.hpp) compiles against the
-    oracle's Frame / KeyFrame / MapPoint stand-ins and links libborb.so: oracle/_ref/libadaptmatch.so exports the same entry
+    oracle's Frame / KeyFrame / MapPoint stand-ins and links libborb.so: oracle/libadaptmatch.so exports the same entry
     points as the verbatim libmatchref.so.  It is EXECUTED on the GPU by tests/test_gpu_adapters.py."""
     import ctypes
-    import pytest
     from oracle import oracle_lib as O
     O.build()
-    so = os.path.join(ROOT, "oracle", "_ref", "libadaptmatch.so")
-    if not os.path.exists(so):
-        pytest.skip("needs the reference tree (DBoW2 FeatureVector) at build time")
+    so = os.path.join(ROOT, "oracle", "libadaptmatch.so")
     lib = ctypes.CDLL(so)
     for name in ("matchref_search_by_projection", "matchref_search_by_projection_last", "matchref_search_by_projection_kf",
                  "matchref_search_by_projection_sim3", "matchref_search_by_bow_kf_f", "matchref_search_by_bow_kf_kf",
@@ -67,16 +64,13 @@ def test_matcher_adapter_library_builds_and_exports_the_reference_entry_points()
 
 def test_keyframe_database_adapter_library_builds_and_fails_loudly_without_a_gpu():
     """integration/KeyFrameDatabase_borb.cc behind the reference's unchanged include/KeyFrameDatabase.h compiles against the
-    dbowshim stand-ins and links libborb.so (oracle/_ref/libadaptdbow.so, same entry points as the verbatim libdbowref.so).
+    dbowshim stand-ins and links libborb.so (oracle/libadaptdbow.so, same entry points as the verbatim libdbowref.so).
     Executed on the GPU by tests/test_gpu_adapters.py; here: the exports, the dependency, and — on a machine without a GPU —
     that a database call surfaces the library's error instead of falling back to anything."""
     import ctypes
-    import pytest
     from oracle import oracle_lib as O
     O.build()
-    so = os.path.join(ROOT, "oracle", "_ref", "libadaptdbow.so")
-    if not os.path.exists(so):
-        pytest.skip("needs the reference tree (DBoW2, KeyFrameDatabase.h) at build time")
+    so = os.path.join(ROOT, "oracle", "libadaptdbow.so")
     lib = ctypes.CDLL(so)
     for name in ("dbowref_voc_load_text", "dbowref_transform", "dbowref_score", "dbowref_detect_candidates", "dbowref_reloc_sequence"):
         assert hasattr(lib, name), name

@@ -1,4 +1,5 @@
-"""CPU: the oracle (restatement AND verbatim reference build) reproduces the committed golden vectors."""
+"""CPU: the oracle (restatement AND verbatim reference build) reproduces the committed golden vectors.  Where the verbatim build
+is absent, what it gave is taken from tests/golden/reference.json (tests/reference_golden.py)."""
 import glob
 import os
 
@@ -6,6 +7,7 @@ import numpy as np
 import pytest
 
 from orb_slam2_b200 import synth
+from tests.reference_golden import ref  # noqa: F401  (fixture)
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -24,12 +26,11 @@ def test_port_reproduces_golden(oracle, path):
 
 
 @pytest.mark.parametrize("path", golden_extract_cases()[:2], ids=os.path.basename)
-def test_verbatim_reference_reproduces_golden(oracle_ref, path):
+def test_verbatim_reference_reproduces_golden(oracle, path, ref):
     g = np.load(path)
     w, h, nf, ini, mn, seed = g["meta"].tolist()
     img = synth.mono_frame(seed, 0, 0, w, h)
-    k, d = oracle_ref.RefExtractor(nf, 1.2, 8, ini, mn)(img)
-    assert np.array_equal(k, g["keypoints"]) and np.array_equal(d, g["descriptors"])
+    ref.expect((g["keypoints"], g["descriptors"]), (lambda: oracle.RefExtractor(nf, 1.2, 8, ini, mn)(img)) if oracle.have_ref() else None)
 
 
 def test_stereo_restatement_reproduces_golden(oracle):
@@ -52,11 +53,9 @@ def test_stereo_restatement_reproduces_golden(oracle):
     assert np.all(dp[m] > 0) and np.all(dp[~m] == -1) and np.all(ur[~m] == -1)
 
 
-def test_stereo_golden_equals_verbatim_frame_cc(oracle):
+def test_stereo_golden_equals_verbatim_frame_cc(oracle, ref):
     """The stereo golden vectors were generated with the restatement; the reference's own Frame.cc, compiled verbatim
     (oracle/_ref/libframeref.so), produces exactly the same numbers on the same inputs."""
-    if not oracle.have_frameref():
-        pytest.skip("oracle/_ref/libframeref.so not built (reference tree absent)")
     g = np.load(os.path.join(GOLD, "stereo_kitti_2000.npz"))
     w, h, nf, seed = g["meta"].tolist()
     bf, fx = g["cam"].tolist()
@@ -64,8 +63,8 @@ def test_stereo_golden_equals_verbatim_frame_cc(oracle):
     EL, ER = oracle.PortExtractor(nf), oracle.PortExtractor(nf)
     kl, dl = EL(L)
     kr, dr = ER(R)
-    ur, dp = oracle.ref_stereo(kl, dl, kr, dr, [EL.level(i) for i in range(8)], [ER.level(i) for i in range(8)], EL.scale, EL.inv_scale, bf, fx)
-    assert np.array_equal(ur, g["u_right"]) and np.array_equal(dp, g["depth"])
+    live = lambda: oracle.ref_stereo(kl, dl, kr, dr, [EL.level(i) for i in range(8)], [ER.level(i) for i in range(8)], EL.scale, EL.inv_scale, bf, fx)
+    ref.expect((g["u_right"], g["depth"]), live if oracle.have_frameref() else None)
 
 
 # ---- matcher golden vectors: outputs of the verbatim-compiled src/ORBmatcher.cc (tests/golden/make_golden_match.py)

@@ -1,6 +1,6 @@
 """GPU: the C++ adapters — the reference-side binding of the drop-in boundary — EXECUTED, not just compiled.
 
-oracle/_ref/libadaptmatch.so = integration/ORBmatcher_borb.cc (the product's drop-in replacement of src/ORBmatcher.cc, i.e.
+oracle/libadaptmatch.so = integration/ORBmatcher_borb.cc (the product's drop-in replacement of src/ORBmatcher.cc, i.e.
 include/borb_matcher_adapters.hpp instantiated for every ORBmatcher method) compiled against the oracle's plain-data
 Frame / KeyFrame / MapPoint stand-ins and wrapped by the SAME C wrappers (oracle/matchref_wrap.cpp) that drive the verbatim
 src/ORBmatcher.cc in libmatchref.so.  Swapping the library under oracle_lib.ref_* therefore sends every call of
@@ -17,11 +17,12 @@ import pytest
 
 from tests import match_fixtures as mf
 from tests import test_oracle_match_ref as T
+from tests.reference_golden import Reference, ref  # noqa: F401  (fixture of the re-collected tests)
 
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-ADAPT_SO = os.path.join(ROOT, "oracle", "_ref", "libadaptmatch.so")
+ADAPT_SO = os.path.join(ROOT, "oracle", "libadaptmatch.so")
 
 
 @pytest.fixture(scope="module", params=["host_view", "resident_frame"])
@@ -29,8 +30,7 @@ def O(oracle, request):
     """host_view: the adapters pass the Frame's host arrays with every call; resident_frame: the wrapper binds a device-resident
     copy of every Frame it builds (borb::adapt::make_resident -> borb_frame_create), so the same fixtures exercise
     borb_frame_view::resident through the adapters (BORB_ADAPT_RESIDENT is read by oracle/matchref_wrap.cpp per call)."""
-    if not os.path.exists(ADAPT_SO):
-        pytest.skip("oracle/_ref/libadaptmatch.so not built (needs the reference tree's DBoW2 FeatureVector at build time)")
+    assert os.path.exists(ADAPT_SO), "build() did not build oracle/libadaptmatch.so"
     saved = oracle.MATCHREF_SO
     oracle.MATCHREF_SO = ADAPT_SO                     # every oracle.ref_* matcher call now runs the ADAPTERS on the GPU
     if request.param == "resident_frame":
@@ -147,7 +147,7 @@ def test_extractor_and_stereo_adapter_program(oracle, tmp_path):
 # ---------------------------------------------------------------------------------------------------------------------------
 # KeyFrameDatabase: integration/KeyFrameDatabase_borb.cc (the drop-in replacement of src/KeyFrameDatabase.cc) behind the real
 # include/KeyFrameDatabase.h, wrapped by the same oracle/dbowref_wrap.cpp as the verbatim build
-ADAPT_DBOW_SO = os.path.join(ROOT, "oracle", "_ref", "libadaptdbow.so")
+ADAPT_DBOW_SO = os.path.join(ROOT, "oracle", "libadaptdbow.so")
 
 
 @pytest.fixture(scope="module")
@@ -155,8 +155,7 @@ def world(oracle, tmp_path_factory):
     """tests/test_oracle_dbow_ref.py's fixture with oracle.DBOWREF_SO pointing at the ADAPTER library: every
     KeyFrameDatabase::add / DetectLoopCandidates / DetectRelocalizationCandidates call of those tests now runs
     adapter -> borb_kfdb_add / borb_kfdb_query (GPU) -> the adapter's host part."""
-    if not os.path.exists(ADAPT_DBOW_SO):
-        pytest.skip("oracle/_ref/libadaptdbow.so not built (needs the reference tree at build time)")
+    assert os.path.exists(ADAPT_DBOW_SO), "build() did not build oracle/libadaptdbow.so"
     saved = oracle.DBOWREF_SO
     oracle.DBOWREF_SO = ADAPT_DBOW_SO
     pv = oracle.PortVocabulary.random(10, 3, 5)
@@ -174,4 +173,4 @@ test_keyframe_database_adapter_equals_reference_source = TD.test_keyframe_databa
 
 
 def test_keyframe_database_adapter_reads_stale_scores_like_the_reference(world):
-    TD.test_relocalization_reads_stale_scores_like_the_reference(world, 21)
+    TD.test_relocalization_reads_stale_scores_like_the_reference(world, 21, Reference("test_relocalization_reads_stale_scores_like_the_reference", {"seed": 21}))
