@@ -55,8 +55,8 @@ struct Geometry {
     int nlevels;
     int w, h;
     int ini_th, min_th;
-    int fast_mode;              // 0: full kernel.  Ablation (borb_debug_set_fast_mode): 1 = TMA tile load only, 2 = + packed reject,
-                                // 3 = + exact scores (no NMS / emit)
+    int fast_mode;              // 0: full kernel.  Ablation (borb_debug_set_fast_mode): 1 = TMA tile load only, 2 = + packed reject
+                                // and pixel queue, 3 = + exact pixel scores (no NMS / emit)
     int fast_blocks;            // FAST CTAs per image (all levels)
     unsigned pyr_image_stride;  // bytes
     unsigned cand_image_stride; // entries

@@ -1,5 +1,6 @@
 """Speed-of-light table for fast_kernel (VERDICT r01 item 3a): the same launch timed with the kernel cut off after
-   mode 1: TMA tile load only   mode 2: + packed reject pass   mode 3: + exact scores (no NMS / emit)   mode 0: full kernel
+   mode 1: TMA tile load only   mode 2: + packed reject and pixel queue   mode 3: + exact pixel scores (no NMS / emit)
+   mode 0: full kernel
 on the bench input (KITTI-shaped 1242x375 stereo pairs, 64 images per launch, 4 rotating batches > L2).  The stage time is the
 CUDA-event time of the `fast_nms` stage on the library's stream (borb_set_timing), mean over --steps launches.
 usage: python tools/fast_ablation.py [--pairs 32] [--steps 40]  -> one JSON line."""
